@@ -50,6 +50,7 @@ NK = READ_LEN - KMER  # 129 informative words per read
 BYTES_PER_READ = READ_LEN + 4 * min(NK, SKETCH)  # 666 (SURVEY 8d)
 METRIC = "mash.Sketch Gbases/s"
 NVLINK_PEER_PEAK_GBS = 770.0  # measured peer-copy bandwidth per direction, B200_PROFILING.md
+DUMP_ROWS = 32768  # --dump-outputs: 32768 x 129 float64 = 34 MB, under 64 MB whatever the world size
 
 
 def parse():
@@ -64,7 +65,15 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--no-pipeline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned: a fixed seeded sample of "
+                         f"{DUMP_ROWS} rows of the [reads][{NK}] uint32 sketch array as DIR/sketches.npy (float64, "
+                         "every uint32 exact) and the read index of each row as DIR/read_index.npy; under torchrun "
+                         "every rank writes its share with a _rank<r> suffix")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 class ClockSampler:
@@ -283,6 +292,21 @@ def barrier(cx):
     if cx.world > 1:
         dist.barrier()
     torch.cuda.synchronize()
+
+
+def dump_outputs(cx, d_out, out_dir):
+    """--dump-outputs: the same rows of the headline step's result on every run with the same --reads
+    (the inputs are counter-based, the sample is seeded), so that two builds can be compared output for output."""
+    import numpy as np
+    import torch
+
+    m = min(cx.n, DUMP_ROWS // cx.world)
+    rows = np.sort(np.random.default_rng(0).choice(cx.n, m, replace=False))
+    got = d_out.view(cx.n, NK)[torch.from_numpy(rows).to(cx.dev)].cpu().numpy().view(np.uint32)
+    suffix = f"_rank{cx.rank}" if cx.world > 1 else ""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"sketches{suffix}.npy"), got.astype(np.float64))
+    np.save(os.path.join(out_dir, f"read_index{suffix}.npy"), (rows + cx.rank * cx.n).astype(np.float64))
 
 
 # ---- e2e ---------------------------------------------------------------------------------------------
@@ -780,6 +804,8 @@ def main():
     rc, want = oracle_ffi.sketch_batch(synth.independent_reads(m, READ_LEN, first_read=first_read), synth.uniform_offsets(m, READ_LEN), KMER, SKETCH, 1, 1)
     got = d_out[: m * NK].cpu().numpy().view(np.uint32).reshape(m, NK)
     headline_parity = all_true(cx, rc == 0 and bool(np.array_equal(got, want[:, :NK])))
+    if args.dump_outputs:
+        dump_outputs(cx, d_out, args.dump_outputs)
 
     e2e = host_bw = e2e_variants = None
     if not args.no_e2e:

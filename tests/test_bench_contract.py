@@ -55,8 +55,40 @@ def test_reference_arm_line(n):
 def test_bench_cli_parses_without_a_gpu():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--help"], capture_output=True, text=True, timeout=120)
     assert out.returncode == 0
-    for flag in ("--gpus", "--steps", "--warmup", "--impl"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--dump-outputs"):
         assert flag in out.stdout
+
+
+@pytest.mark.gpu
+def test_dump_outputs_repeat_and_match_the_oracle(tmp_path, oracle):
+    """--dump-outputs: the same files, bit for bit, from two runs with different --steps; --steps sets the timed
+    launches; every checked row is the oracle's sketch of the read its index names."""
+    import numpy as np
+
+    from poly_b200 import synth
+
+    per_step = []
+    for steps in (2, 3):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", str(steps), "--warmup", "1",
+                              "--reads", "100000", "--no-cpu", "--no-e2e", "--no-secondary", "--dump-outputs", str(tmp_path / str(steps))],
+                             capture_output=True, text=True, timeout=600)
+        assert out.returncode == 0, out.stderr[-3000:]
+        d = json.loads(out.stdout.strip().splitlines()[-1])
+        assert d["steps"] == steps and d["gpu_launches"] % steps == 0 and all(d["parity"].values())
+        per_step.append(d["gpu_launches"] // steps)
+    assert per_step[0] == per_step[1] > 0
+    names = sorted(p.name for p in (tmp_path / "2").iterdir())
+    assert names == ["read_index.npy", "sketches.npy"]
+    assert sum(p.stat().st_size for p in (tmp_path / "2").iterdir()) <= 64 << 20
+    for name in names:
+        assert np.array_equal(np.load(tmp_path / "2" / name), np.load(tmp_path / "3" / name))
+    sk, idx = np.load(tmp_path / "2" / "sketches.npy"), np.load(tmp_path / "2" / "read_index.npy")
+    assert sk.dtype == idx.dtype == np.float64 and sk.shape == (32768, 129) and idx.shape == (32768,)
+    assert np.all(np.diff(idx) > 0) and idx[0] >= 0 and idx[-1] < 100000
+    for row in range(0, len(idx), 1024):
+        read = synth.independent_reads(1, 150, first_read=int(idx[row]))
+        rc, want = oracle.sketch_batch(read, synth.uniform_offsets(1, 150), 21, 1000, variant=1)
+        assert rc == 0 and np.array_equal(sk[row], want[0, :129].astype(np.float64)), row
 
 
 def test_documented_numbers_trace_to_the_record_lines():

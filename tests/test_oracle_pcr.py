@@ -1,12 +1,11 @@
 """Pins the CPU restatement of pcr.Simulate (tests/pcr_util.py, Tm from oracle/) on the expectations of
 the reference's own tests: primers/pcr/example_test.go:10-36,58-69 and pcr_test.go:13-101."""
-import re
+import json
+import os
 
 import pytest
 
 import pcr_util as P
-
-REF_EXAMPLE = "/root/reference/primers/pcr/example_test.go"
 
 
 def test_reference_expectations():
@@ -15,16 +14,14 @@ def test_reference_expectations():
         assert ok(fr, err), primers
 
 
-@pytest.mark.skipif(not __import__("os").path.exists(REF_EXAMPLE), reason="reference only exists in the build container")
 def test_constants_equal_the_reference_test_files():
-    ex = open(REF_EXAMPLE).read()
-    want = re.search(r"// Output: \[(\w+)\]", ex).group(1)
-    assert P.FULL_AMPLICON == want
-    assert P.GENE.decode() == re.search(r'gene := "(\w+)"', ex).group(1)
-    assert P.BAD_FRAGMENT.decode() == re.search(r'badFragment := "(\w+)"', ex).group(1)
-    t = open("/root/reference/primers/pcr/pcr_test.go").read()
-    assert P.CIRCULAR_TARGET == re.search(r'targetFragment := "(\w+)"', t).group(1)
-    assert P.FULL_AMPLICON == re.search(r'want := "(\w+)"', t).group(1)
+    """The strings of the reference's example_test.go / pcr_test.go, as tests/golden/make_pcr_goldens.py stored them."""
+    g = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "pcr_goldens.json")))
+    assert P.FULL_AMPLICON == g["example_simulate_output"]
+    assert P.GENE.decode() == g["example_gene"]
+    assert P.BAD_FRAGMENT.decode() == g["example_bad_fragment"]
+    assert P.CIRCULAR_TARGET == g["circular_target_fragment"]
+    assert P.FULL_AMPLICON == g["issue279_want"]
 
 
 def test_minimal_length_quirks():
