@@ -10,7 +10,6 @@
 //                           owns a TILE x TILE block of pairs with both sketch tiles
 //                           staged in shared memory.
 #include <algorithm>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -290,7 +289,7 @@ int distance_plan_create(const uint32_t *d_sk, uint64_t n, int s, cudaStream_t s
     uint32_t n_unsorted = 1;
     PG_CUDA(cudaMemcpyAsync(&n_unsorted, d_unsorted, 4, cudaMemcpyDeviceToHost, st));
     PG_CUDA(cudaStreamSynchronize(st));
-    if (n_unsorted == 0 && !getenv("PG_K3_PAIRWISE")) return join_build(d_sk, n, s, st, &plan->join);
+    if (n_unsorted == 0) return join_build(d_sk, n, s, st, &plan->join);
     return PG_OK;
 }
 

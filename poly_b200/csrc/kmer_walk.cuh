@@ -12,8 +12,6 @@
 //   sb                     byte pointer: the tail byte of k-mer i is sb[i]      (LUT only)
 //   lut_stride, lut_base   shared-memory tail table (256 x kmix(byte)); the stride (4) is a
 //                          runtime value so byte*4 + base stays an IMAD on the FMA pipe
-//   ROTF, rotmul           number of leading body rounds whose rotate runs on the FMA pipe (0 = none) and the
-//                          runtime multiplier 8192 they use (murmur3.cuh, mm3_round_fma)
 //   my_out, i, nk          hashes of k-mers i .. i+3 go to my_out[i ..]; CHECKED guards i+r < nk
 #pragma once
 #include <stdint.h>
@@ -50,9 +48,9 @@ static __device__ __align__(16) const KmixTable g_kmix_byte = make_kmix_table();
         w[3] = __funnelshift_r(w_cur, w_nxt, 24);                                              \
         uint32_t h[4];                                                                         \
         _Pragma("unroll") for (int r = 0; r < 4; ++r) {                                        \
-            uint32_t x = ROTF > 0 ? mm3_round_fma(0u, ring[r][U], rotmul) : mm3_round0(ring[r][U]); \
+            uint32_t x = mm3_round0(ring[r][U]);                                               \
             _Pragma("unroll") for (int j = 1; j < NB; ++j)                                     \
-                x = j < ROTF ? mm3_round_fma(x, ring[r][((U) + j) % NB], rotmul) : mm3_round(x, ring[r][((U) + j) % NB]); \
+                x = mm3_round(x, ring[r][((U) + j) % NB]);                                     \
             if (LUT) x ^= lds_u32(sb[i + r] * lut_stride + lut_base);                          \
             else if (TAIL) x ^= mm3_kmix(w[r] & TAILMASK);                                     \
             x ^= (uint32_t)K;                                                                  \

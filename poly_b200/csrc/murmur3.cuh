@@ -31,15 +31,6 @@ __device__ __forceinline__ uint32_t mm3_round(uint32_t h, uint32_t kq) {
     h = rotl32(h, 13);
     return h * 5u + MM3_N;
 }
-// The same round with the rotate on the FMA pipe: (hi, lo) = h * 2^13 as a 64-bit product
-// (IMAD.WIDE; rotmul == 8192 arrives as a kernel argument so that ptxas cannot turn the multiply back
-// into a shift), rotl(h, 13) == lo + hi (disjoint bits), so rotl * 5 + N == lo * 5 + (hi * 5 + N):
-// three FMA-pipe instructions instead of one ALU-pipe SHF + one IMAD.  A/B experiment (PG_K1_ROTFMA).
-__device__ __forceinline__ uint32_t mm3_round_fma(uint32_t h, uint32_t kq, uint32_t rotmul) {
-    h ^= kq;
-    const uint64_t w = (uint64_t)h * (uint64_t)rotmul;
-    return (uint32_t)w * 5u + ((uint32_t)(w >> 32) * 5u + MM3_N);
-}
 __device__ __forceinline__ uint32_t mm3_fmix(uint32_t h) {
     h ^= h >> 16;
     h *= 0x85ebca6bu;

@@ -2,7 +2,7 @@
 // written positionally (/root/reference/search/mash/mash.go:73-84).
 //
 // Fast path (fixed-length reads, k in the instantiated set, compact output):
-//   * one CTA = one tile of R reads; the R*L input bytes are contiguous in HBM and are
+//   * one CTA = one warp = one tile of 32 reads; the 32*L input bytes are contiguous in HBM and are
 //     brought in by ONE 1-D TMA bulk copy (cp.async.bulk + mbarrier; SASS UBLKCP);
 //   * one THREAD per read walks the read 4 bytes per step.  The murmur3 block pre-mix
 //     K(p) = rotl(w(p)*c1,15)*c2 of the 4 bytes at position p is computed ONCE and kept
@@ -22,7 +22,6 @@
 // Generic path (any k >= 0, ragged reads, any row stride): one warp per read, every
 // k-mer hashed from scratch.  Slower, same results.
 #include <algorithm>
-#include <cstdlib>
 
 #include "common.cuh"
 #include "murmur3.cuh"
@@ -32,56 +31,48 @@
 namespace pg {
 
 // ---- K1 fast path ----------------------------------------------------------------
-// smem: [0,16) mbarrier | in tile (R*L bytes + 16 B over-read pad, 16-B rounded) | out tile
+// smem: in tile (32*L bytes + 16 B over-read pad, 16-B rounded) | out tile [32][nk]
 // (+ 1 KB static table when k % 4 == 1)
-__host__ __device__ inline uint32_t k1_in_bytes(uint32_t R, uint32_t L) {
-    return (R * L + 16u + 15u) & ~15u;
+__host__ __device__ inline uint32_t k1_in_bytes(uint32_t L) {
+    return (32u * L + 16u + 15u) & ~15u;
 }
 
 // lut_stride == 4 arrives as a kernel argument so that the table address byte*4 + base
 // stays an IMAD (FMA pipe) instead of being strength-reduced to LEA (ALU pipe).
-template <int K, int R, int ROTF = 0>
-__global__ void __launch_bounds__(R)
+template <int K>
+__global__ void __launch_bounds__(32)
 sketch_fill_uniform_kernel(const uint8_t *__restrict__ bases, const SketchDst dst,
-                           uint32_t L, uint32_t nk, uint32_t lut_stride, uint32_t rotmul) {
+                           uint32_t L, uint32_t nk, uint32_t lut_stride) {
     constexpr int NB = K / 4;    // 4-byte body blocks per k-mer
     constexpr int TAIL = K % 4;  // tail bytes per k-mer
     constexpr uint32_t TAILMASK = TAIL == 1 ? 0xffu : TAIL == 2 ? 0xffffu : 0xffffffu;
     constexpr bool LUT = TAIL == 1;
     static_assert(NB >= 1, "fast path needs k >= 4");
 
-    // A CTA holds R/32 warps; every warp owns one tile of 32 reads with its own mbarrier, input
-    // and output staging and bulk store, so the warps of a CTA never wait for each other (they
-    // only share the 1 KB tail table: with R == 64 ten warps fit an SM instead of nine).
-    constexpr int NW = R / 32;
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ __align__(16) uint32_t s_lut[LUT ? 256 : 4];
-    __shared__ __align__(8) uint64_t s_bar[NW + 1];  // [w]: tile of warp w; [NW]: the table
-    const uint32_t wid = threadIdx.x >> 5;
-    const uint32_t tid = threadIdx.x & 31u;  // lane == read within the warp's tile
-    const uint32_t warp_smem = k1_in_bytes(32, L) + 32u * nk * 4u;
-    uint8_t *s_in = smem + wid * warp_smem;
-    uint32_t *s_out = reinterpret_cast<uint32_t *>(s_in + k1_in_bytes(32, L));
-    uint64_t *bar = &s_bar[wid];
+    __shared__ __align__(8) uint64_t s_bar[2];  // [0]: the tile; [1]: the table
+    uint8_t *s_in = smem;
+    uint32_t *s_out = reinterpret_cast<uint32_t *>(smem + k1_in_bytes(L));
 
-    const uint64_t tile = (uint64_t)blockIdx.x * NW + wid;
+    const uint32_t tid = threadIdx.x;  // lane == read within the tile
+    const uint64_t tile = blockIdx.x;
     const uint32_t in_bytes = 32u * L;  // multiple of 16 (host guarantees)
 
-    if (threadIdx.x == 0) {
-        for (int w = 0; w <= NW; ++w) mbar_init(&s_bar[w], 1);
+    if (tid == 0) {
+        mbar_init(&s_bar[0], 1);
+        mbar_init(&s_bar[1], 1);
         fence_mbar_init();
+        mbar_expect_tx(&s_bar[0], in_bytes);
+        bulk_g2s(s_in, bases + tile * in_bytes, in_bytes, &s_bar[0]);
         if (LUT) {
-            mbar_expect_tx(&s_bar[NW], 1024u);
-            bulk_g2s(s_lut, &g_kmix_byte, 1024u, &s_bar[NW]);
+            mbar_expect_tx(&s_bar[1], 1024u);
+            bulk_g2s(s_lut, &g_kmix_byte, 1024u, &s_bar[1]);
         }
     }
-    __syncthreads();  // barrier init visible to everyone (the only CTA-wide barrier)
-    if (tid == 0) {
-        mbar_expect_tx(bar, in_bytes);
-        bulk_g2s(s_in, bases + tile * in_bytes, in_bytes, bar);
-    }
-    mbar_wait(bar, 0);
-    if (LUT) mbar_wait(&s_bar[NW], 0);
+    __syncwarp();  // barrier init visible to every lane
+    mbar_wait(&s_bar[0], 0);
+    if (LUT) mbar_wait(&s_bar[1], 0);
 
     // my read: bytes [tid*L, tid*L+L) of the tile, realigned to words on the fly
     const uint32_t b0 = tid * L;
@@ -154,8 +145,6 @@ sketch_fill_ragged_kernel(const uint8_t *__restrict__ bases, const uint64_t *__r
     constexpr int TAIL = K % 4;
     constexpr uint32_t TAILMASK = TAIL == 1 ? 0xffu : TAIL == 2 ? 0xffffu : 0xffffffu;
     constexpr bool LUT = TAIL == 1;
-    constexpr int ROTF = 0;
-    const uint32_t rotmul = 0;
     static_assert(NB >= 1, "fast path needs k >= 4");
 
     extern __shared__ __align__(128) uint8_t smem[];
@@ -289,33 +278,22 @@ sketch_fill_generic_kernel(const uint8_t *__restrict__ bases, const uint64_t *__
 }
 
 // ---- launchers -------------------------------------------------------------------
-template <int K, int R, int ROTF = 0>
+template <int K>
 static int launch_k1(const uint8_t *d_bases, uint64_t n_tiles, uint32_t L, uint32_t nk,
                      const SketchDst &dst, cudaStream_t st) {
-    const size_t smem = (size_t)(R / 32) * (k1_in_bytes(32, L) + (size_t)32 * nk * 4);
-    { const int rc_ = func_smem((const void *)sketch_fill_uniform_kernel<K, R, ROTF>, smem); if (rc_ != PG_OK) return rc_; }
-    sketch_fill_uniform_kernel<K, R, ROTF><<<(unsigned)n_tiles, R, smem, st>>>(d_bases, dst, L, nk, 4u, 8192u);
+    const size_t smem = k1_in_bytes(L) + (size_t)32 * nk * 4;
+    { const int rc_ = func_smem((const void *)sketch_fill_uniform_kernel<K>, smem); if (rc_ != PG_OK) return rc_; }
+    sketch_fill_uniform_kernel<K><<<(unsigned)n_tiles, 32, smem, st>>>(d_bases, dst, L, nk, 4u);
     PG_LAUNCH_CHECK("sketch_fill_uniform_kernel");
     return PG_OK;
 }
 
-template <int R>
 static int dispatch_k1(int k, const uint8_t *d_bases, uint64_t n_tiles, uint32_t L, uint32_t nk,
                        const SketchDst &dst, cudaStream_t st, bool *handled) {
     *handled = true;
-    // A/B knob: PG_K1_ROTFMA=n moves the rotate of the first n body rounds to the FMA pipe (k = 21 only)
-    static const int rotf = [] { const char *e = getenv("PG_K1_ROTFMA"); return e ? atoi(e) : 0; }();
-    if (k == 21 && R == 32 && rotf > 0) {
-        switch (rotf) {
-            case 1: return launch_k1<21, 32, 1>(d_bases, n_tiles, L, nk, dst, st);
-            case 2: return launch_k1<21, 32, 2>(d_bases, n_tiles, L, nk, dst, st);
-            case 3: return launch_k1<21, 32, 3>(d_bases, n_tiles, L, nk, dst, st);
-            default: return launch_k1<21, 32, 5>(d_bases, n_tiles, L, nk, dst, st);
-        }
-    }
     switch (k) {
 #define PG_K1_CASE(KK) \
-    case KK: return launch_k1<KK, R>(d_bases, n_tiles, L, nk, dst, st);
+    case KK: return launch_k1<KK>(d_bases, n_tiles, L, nk, dst, st);
         PG_K1_CASE(11) PG_K1_CASE(13) PG_K1_CASE(15) PG_K1_CASE(16) PG_K1_CASE(17) PG_K1_CASE(19)
         PG_K1_CASE(21) PG_K1_CASE(23) PG_K1_CASE(24) PG_K1_CASE(25) PG_K1_CASE(27) PG_K1_CASE(29)
         PG_K1_CASE(31) PG_K1_CASE(32)
@@ -323,9 +301,6 @@ static int dispatch_k1(int k, const uint8_t *d_bases, uint64_t n_tiles, uint32_t
     default: *handled = false; return PG_OK;
     }
 }
-
-// warps (= independent 32-read tiles) per CTA
-constexpr int K1_WARPS = 1;
 
 static int launch_fill_generic(const uint8_t *d_bases, const uint64_t *d_offsets, uint32_t ulen,
                                uint64_t n_reads, uint64_t first_read, int k, int s, uint32_t flags,
@@ -358,23 +333,19 @@ int launch_sketch_uniform(const uint8_t *d_bases, uint64_t n_reads, uint32_t L, 
     bool aligned = ((uintptr_t)d_bases % 16 == 0) && ((uintptr_t)d_out % 16 == 0);
     if (extra)
         for (int p = 0; p < extra->n; ++p) aligned = aligned && ((uintptr_t)extra->ptr[p] % 16 == 0);
-    // tiles of 32 reads; a CTA runs NW of them on NW independent warps (PG_K1_WARPS=1|2, A/B knob)
-    static const int nw_pref = [] { const char *e = getenv("PG_K1_WARPS"); return e ? atoi(e) : K1_WARPS; }();
-    const size_t smem1 = k1_in_bytes(32, L) + (size_t)32 * nk * 4;
+    // tiles of 32 reads, one per CTA
+    const size_t smem1 = k1_in_bytes(L) + (size_t)32 * nk * 4;
     if (compact && aligned && nk > 0 && (32 * (uint64_t)L) % 16 == 0 && smem1 <= 100 * 1024 && n_reads >= 32) {
         const uint64_t tiles = n_reads / 32;
         bool handled = false;
         uint64_t t0 = 0;
         while (t0 < tiles) {
-            const int nw = (nw_pref == 2 && tiles - t0 >= 2) ? 2 : 1;
-            // grid.x limit; with 2 warps per CTA an odd last tile takes a 1-warp launch
-            const uint64_t nt = std::min<uint64_t>((tiles - t0) / nw, 0x7fffffffull) * nw;
+            const uint64_t nt = std::min<uint64_t>(tiles - t0, 0x7fffffffull);  // grid.x limit
             SketchDst dst;
             dst.n = extra ? extra->n : 1;
             for (int p = 0; p < dst.n; ++p)
                 dst.ptr[p] = (extra ? extra->ptr[p] : d_out) + t0 * 32 * (uint64_t)nk;
-            int rc = nw == 2 ? dispatch_k1<64>(k, d_bases + t0 * 32 * (uint64_t)L, nt / 2, L, nk, dst, st, &handled)
-                             : dispatch_k1<32>(k, d_bases + t0 * 32 * (uint64_t)L, nt, L, nk, dst, st, &handled);
+            int rc = dispatch_k1(k, d_bases + t0 * 32 * (uint64_t)L, nt, L, nk, dst, st, &handled);
             if (rc != PG_OK) return rc;
             if (!handled) break;
             t0 += nt;

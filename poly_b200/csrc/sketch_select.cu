@@ -449,8 +449,6 @@ sketch_select_walk_kernel(const uint8_t *__restrict__ bases, const uint64_t *__r
     constexpr uint32_t TAILMASK = TAIL == 1 ? 0xffu : TAIL == 2 ? 0xffffu : 0xffffffu;
     constexpr bool LUT = TAIL == 1;
     constexpr uint32_t k = K;
-    constexpr int ROTF = 0;
-    const uint32_t rotmul = 0;
     static_assert(NB >= 1 && K <= 32, "walk path: 4 <= k <= 32");
     static_assert(SELW_SEG % 4 == 0, "a segment is a whole number of word steps");
 
@@ -739,7 +737,7 @@ select_merge_kernel(const uint32_t *__restrict__ part, const uint32_t *__restric
 // the mean -- and whether it did is CHECKED, never assumed: a row whose admitted count is < s (few
 // distinct k-mers) or exceeds its buffer (heavy duplication below T) is redone by the exact streaming
 // kernel above (retry list built on the device, no host round trip).  So:
-//   A. sketch_thresh_walk_kernel<K, RARE, ROLLED>: one WARP per work item (<= 8 chunks of 32 x SEG
+//   A. sketch_thresh_walk_kernel<K, RARE>: one WARP per work item (<= 8 chunks of 32 x SEG
 //      positions of one row, SeltGeom<K>; long sequences become many items, so there is no host-side
 //      slicing and no merge pass).  Chunks arrive by double-buffered 1-D TMA bulk copies; lane l walks SEG
 //      consecutive k-mers with the register ring of kmer_walk.cuh (one ring prologue per SEG k-mers
@@ -801,7 +799,7 @@ __device__ __forceinline__ void strip_advance_if_le(uint32_t &saddr, uint32_t h,
         }                                                                                \
     }
 
-template <int K, bool RARE, bool ROLLED>
+template <int K, bool RARE>
 __global__ void __launch_bounds__(32)
 sketch_thresh_walk_kernel(const uint8_t *__restrict__ bases, const uint64_t *__restrict__ offsets, uint32_t uniform_len,
                           uint64_t row0, uint64_t n_rows, uint32_t items_per_row, uint32_t s, uint32_t mu, uint32_t cap,
@@ -811,8 +809,7 @@ sketch_thresh_walk_kernel(const uint8_t *__restrict__ bases, const uint64_t *__r
     constexpr uint32_t TAILMASK = TAIL == 1 ? 0xffu : TAIL == 2 ? 0xffffu : 0xffffffu;
     constexpr bool LUT = TAIL == 1;
     constexpr uint32_t k = K;
-    constexpr int ROTF = 0;
-    const uint32_t rotmul = 0;
+    constexpr bool ROLLED = SELT_ROLLED_DEFAULT(K);
     static_assert(NB >= 1 && K <= 32, "walk path: 4 <= k <= 32");
     constexpr int SELT_SEG = SeltGeom<K>::SEG, SELT_CHUNK = SeltGeom<K>::CHUNK, SELT_STAGE_BYTES = SeltGeom<K>::STAGE;
 
@@ -1270,11 +1267,7 @@ static int launch_select_thresh(const uint8_t *d_bases, const uint64_t *d_offset
     // admission probability of the longest rows: below 1/512 a warp step (128 hashes) admits something a quarter of the time
     const uint32_t tm1_u = d_offsets ? 0u : selt_threshold_m1(nmax, mu);  // every row of a fixed-length batch has n == nmax
     const bool rare = (uint64_t)mu * 512 < nmax;
-    // PG_K2T_ROLLED=1: 3-step loop body with the ring rotated by register moves, =0: NB-step body (A/B and test knob)
-    const int rolled_env = [] { const char *e = getenv("PG_K2T_ROLLED"); return e ? atoi(e) : -1; }();
-    const bool rolled = K / 4 >= 3 && (rolled_env >= 0 ? rolled_env != 0 : SELT_ROLLED_DEFAULT(K));  // the 3-step group needs NB >= 3
-    const void *walk_fn = rare ? (rolled ? (const void *)sketch_thresh_walk_kernel<K, true, true> : (const void *)sketch_thresh_walk_kernel<K, true, false>)
-                               : (rolled ? (const void *)sketch_thresh_walk_kernel<K, false, true> : (const void *)sketch_thresh_walk_kernel<K, false, false>);
+    const void *walk_fn = rare ? (const void *)sketch_thresh_walk_kernel<K, true> : (const void *)sketch_thresh_walk_kernel<K, false>;
     { const int rc_ = func_smem(walk_fn, smem_a); if (rc_ != PG_OK) return rc_; }
     // batch width of the select: fewest load slots for a typical row (mu + 2.5 sigma candidates), ties to the wider batch
     const uint32_t typ = mu + (uint32_t)(2.5 * sqrt((double)mu));
@@ -1286,16 +1279,12 @@ static int launch_select_thresh(const uint8_t *d_bases, const uint64_t *d_offset
             if (slots <= best) { best = slots; sel_u = u; }
         }
     }
-    const int sel_u_env = [] { const char *e = getenv("PG_K2T_SEL_U"); return e ? atoi(e) : 0; }();      // A/B and test knobs, read per call
-    const int sel_mul_env = [] { const char *e = getenv("PG_K2T_SEL_MUL"); return e ? atoi(e) : -1; }();
-    if (sel_u_env == 3 || sel_u_env == 4 || sel_u_env == 5 || sel_u_env == 6 || sel_u_env == 8) sel_u = sel_u_env;
     // bucket function: the plain shift when it uses >= 3/4 of the 2048 buckets (fixed-length batch: T known here)
     bool sel_mul = true;
     if (!d_offsets) {
         const uint32_t tb = 32u - (uint32_t)__builtin_clz(tm1_u | 1u);
         sel_mul = ((tm1_u >> (tb > 11u ? tb - 11u : 0u)) + 1u) < 1536u;
     }
-    if (sel_mul_env >= 0) sel_mul = sel_mul_env != 0;
 #define PG_SEL_FN(U_) (sel_mul ? (const void *)sketch_thresh_select_kernel<U_, true> : (const void *)sketch_thresh_select_kernel<U_, false>)
     const void *sel_fn = sel_u == 3 ? PG_SEL_FN(3) : sel_u == 4 ? PG_SEL_FN(4) : sel_u == 5 ? PG_SEL_FN(5) : sel_u == 6 ? PG_SEL_FN(6) : PG_SEL_FN(8);
 #undef PG_SEL_FN
@@ -1317,13 +1306,11 @@ static int launch_select_thresh(const uint8_t *d_bases, const uint64_t *d_offset
     for (uint64_t r0 = 0; r0 < n_reads; r0 += group) {
         const uint64_t rows = std::min(group, n_reads - r0);
         PG_CUDA(cudaMemsetAsync(d_cnt, 0, rows * 4, st));
-#define PG_LAUNCH_WALK(RARE_, ROLLED_)                                                                                     \
-    sketch_thresh_walk_kernel<K, RARE_, ROLLED_><<<(unsigned)(rows * ipr), 32, smem_a, st>>>(d_bases, d_offsets, read_len, r0, rows, \
-                                                                                            (uint32_t)ipr, (uint32_t)s, mu, cap, d_cand, d_cnt, 4u, tm1_u)
-        if (rare && rolled) PG_LAUNCH_WALK(true, true);
-        else if (rare) PG_LAUNCH_WALK(true, false);
-        else if (rolled) PG_LAUNCH_WALK(false, true);
-        else PG_LAUNCH_WALK(false, false);
+#define PG_LAUNCH_WALK(RARE_)                                                                                              \
+    sketch_thresh_walk_kernel<K, RARE_><<<(unsigned)(rows * ipr), 32, smem_a, st>>>(d_bases, d_offsets, read_len, r0, rows, \
+                                                                                   (uint32_t)ipr, (uint32_t)s, mu, cap, d_cand, d_cnt, 4u, tm1_u)
+        if (rare) PG_LAUNCH_WALK(true);
+        else PG_LAUNCH_WALK(false);
 #undef PG_LAUNCH_WALK
         PG_LAUNCH_CHECK("sketch_thresh_walk_kernel");
         const uint64_t blocks = std::min<uint64_t>(rows, (uint64_t)sm_count() * std::max(per_sm, 1));
@@ -1355,17 +1342,13 @@ template <int K>
 static int launch_select_auto(const uint8_t *d_bases, const uint64_t *d_offsets, uint32_t read_len, uint64_t max_read_len, uint64_t n_reads, int s,
                               uint32_t P, uint32_t *d_out, uint64_t row_stride, uint32_t *d_count, int32_t *d_status,
                               cudaStream_t st, const SketchDst &ex) {
-    static const bool no_slices = [] { const char *e = getenv("PG_K2_NO_SLICES"); return e && atoi(e) != 0; }();
-    static const bool no_thresh = [] { const char *e = getenv("PG_K2_NO_THRESH"); return e && atoi(e) != 0; }();  // A/B knob
-    if (!no_thresh) {
-        bool handled = false;
-        const int rc = launch_select_thresh<K>(d_bases, d_offsets, read_len, max_read_len, n_reads, s, P, d_out, row_stride, d_count, d_status, st,
-                                               ex, &handled);
-        if (rc != PG_OK || handled) return rc;
-    }
-    if (ex.n == 0 && !no_slices) {
+    bool handled = false;
+    int rc = launch_select_thresh<K>(d_bases, d_offsets, read_len, max_read_len, n_reads, s, P, d_out, row_stride, d_count, d_status, st, ex,
+                                     &handled);
+    if (rc != PG_OK || handled) return rc;
+    if (ex.n == 0) {
         bool sliced = false;
-        const int rc = try_select_sliced<K>(d_bases, d_offsets, read_len, n_reads, s, P, d_out, row_stride, d_count, d_status, st, &sliced);
+        rc = try_select_sliced<K>(d_bases, d_offsets, read_len, n_reads, s, P, d_out, row_stride, d_count, d_status, st, &sliced);
         if (rc != PG_OK || sliced) return rc;
     }
     return launch_select_walk<K>(d_bases, d_offsets, read_len, n_reads, s, P, d_out, row_stride, d_count, d_status, st, ex);
@@ -1391,9 +1374,8 @@ int launch_sketch_select(const uint8_t *d_bases, const uint64_t *d_offsets, uint
     uint32_t P = 1;
     while (P < (uint32_t)std::max(s, 1)) P <<= 1;
     if (P < 2) P = 2;
-    // K2w (register-ring walk) for the instantiated k; PG_K2_GENERIC=1 forces the generic kernel (A/B knob)
-    static const bool force_generic = [] { const char *e = getenv("PG_K2_GENERIC"); return e && atoi(e) != 0; }();
-    if (!force_generic && (size_t)s * 8 + 56 * 1024 <= 227 * 1024) {  // shared memory of the walk kernel
+    // K2t / K2w (register-ring walks) for the instantiated k
+    if ((size_t)s * 8 + 56 * 1024 <= 227 * 1024) {  // shared memory of the walk kernel
         switch (k) {
 #define PG_K2W_CASE(KK) \
     case KK: return launch_select_auto<KK>(d_bases, d_offsets, read_len, max_read_len, n_reads, s, P, d_out, row_stride, d_count, d_status, st, ex);

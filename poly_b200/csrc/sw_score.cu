@@ -13,7 +13,6 @@
 // the outer loop; the reported error (first failing cell in row-major order,
 // align.go:188-191) does, and is resolved per orientation at the end.
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 #include <limits>
 #include <type_traits>
@@ -486,8 +485,7 @@ int launch_sw_score(const uint8_t *d_q, const uint64_t *d_qoff, uint64_t nq, uin
                                            (long double)std::max(amax, agap);
     if (bound < 2.0e9L) {
         // two queries per register (2 x int16) when a local alignment's values stay below 2^14 and gap <= 0
-        static const bool no_x2 = [] { const char *e = getenv("PG_SW_NO_X2"); return e && atoi(e) != 0; }();  // A/B knob
-        const bool x2_ok = !global && gap <= 0 && bound < 16000.0L && agap < 16000 && nq >= 2 && !no_x2;
+        const bool x2_ok = !global && gap <= 0 && bound < 16000.0L && agap < 16000 && nq >= 2;
         return run_sw<int>(p, max_qlen, lut_q, lut_t, tab_qt, gap, d_score, d_err, d_errpos, st, x2_ok);
     }
     return run_sw<long long>(p, max_qlen, lut_q, lut_t, tab_qt, gap, d_score, d_err, d_errpos, st);

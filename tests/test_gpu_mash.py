@@ -136,7 +136,7 @@ def test_select_regime_long_reads_with_pruning(gpu, oracle):
         seqs = [bytes(rng.choice(list(b"ACGT"), size=l).astype(np.uint8)) for l in lens]
         seqs.append(bytes(rng.choice(list(b"AC"), size=70_001).astype(np.uint8)))
         seqs.append(b"ACG" * 20_000)
-        if s == 1000:  # a genome-sized sequence: cut into slices, sketched in parallel, merged
+        if s == 1000:  # a genome-sized sequence: one row spread over many work items of the threshold walk
             seqs.append(bytes(rng.choice(list(b"ACGT"), size=2_500_003).astype(np.uint8)))
             seqs += [bytes(rng.choice(list(b"ACGT"), size=int(l)).astype(np.uint8)) for l in rng.integers(0, 3000, 40)]
         bases, offsets = mash.flatten(seqs)
@@ -293,10 +293,11 @@ def _oracle_same_matrix(oracle, sk, rows):
     return out
 
 
-def test_distance_join_multiset_and_skew(gpu, oracle, monkeypatch):
+def test_distance_join_multiset_and_skew(gpu, oracle):
     """All-ascending inputs take the inverted-index join (distance_join.cu): duplicates inside a
     sketch (multiset min-count), identical sketches, values piled into one bucket, row blocks;
-    and the pairwise kernel (PG_K3_PAIRWISE=1) must agree with it."""
+    and the same sets with one non-ascending row appended take the pairwise kernel, which must
+    agree with the oracle on the ascending rows as well."""
     rng = np.random.default_rng(21)
     cases = []
     # (a) low-complexity reads: many repeated k-mers -> duplicate hashes inside each sketch
@@ -320,8 +321,9 @@ def test_distance_join_multiset_and_skew(gpu, oracle, monkeypatch):
         assert np.array_equal(dist, 1 - want / float(sk.shape[1]))
         s2, _ = mash.distance_block(sk, 3, n - 2)
         assert np.array_equal(s2, want[3:n - 2])
-    monkeypatch.setenv("PG_K3_PAIRWISE", "1")
     for sk in cases:
+        sk = np.concatenate([sk, sk[1:2, ::-1]])  # a descending copy of row 1
+        assert (sk[-1, 1:] < sk[-1, :-1]).any()
         same, _ = mash.distance_block(sk)
         assert np.array_equal(same, _oracle_same_matrix(oracle, sk, range(len(sk))))
 
@@ -435,27 +437,26 @@ def test_select_threshold_path(gpu, oracle, monkeypatch):
     retry list hands to the exact streaming kernel.  Everything bit-exact against the oracle."""
     rng = np.random.default_rng(77)
     monkeypatch.setenv("PG_K2T_GROUP_ROWS", "7")
+    # Between them the cases (and the ragged batch below) run every select-stage variant, (batch width U, bucket
+    # function) as launch_select_thresh picks them from k, s and L:
+    #   (3, shift) k = 32          (3, mul) k = 16, k = 11       (4, shift) s = 517, L = 539   (4, mul) s = 517, L = 1055
+    #   (5, shift) k = 31          (5, mul) s = 733              (6, shift) k = 21, s = 1000   (6, mul) the ragged batch
+    #   (8, shift) s = 1185        (8, mul) k = 24
+    # and the walk with rare admissions (fewer than 1 in 512 hashes, the last case) next to the common one.
     cases = [(21, 1000, 40_000, 20), (31, 2000, 10_000, 40), (16, 64, 5_000, 33), (21, 1000, 1021 + 21, 9), (21, 1000, 1300, 9),
-             (24, 5000, 30_000, 5), (32, 3, 9_000, 12), (11, 500, 2176 * 8 + 11 + 1, 6), (28, 300, 7_013, 8)]
-    # both bucket functions of the select stage and both loop shapes of the walk, on every case
-    for knobs in ({}, {"PG_K2T_SEL_MUL": "0", "PG_K2T_ROLLED": "0", "PG_K2T_SEL_U": "3"}, {"PG_K2T_SEL_MUL": "1", "PG_K2T_ROLLED": "1", "PG_K2T_SEL_U": "8"}):
-        for name in ("PG_K2T_SEL_MUL", "PG_K2T_ROLLED", "PG_K2T_SEL_U"):
-            monkeypatch.delenv(name, raising=False)
-        for name, v in knobs.items():
-            monkeypatch.setenv(name, v)
-        for k, s, L, n in cases:
-            reads = rng.choice(list(b"ACGT"), size=n * L).astype(np.uint8).reshape(n, L)
-            reads[1] = ord("A")                                                   # homopolymer: one distinct hash
-            reads[2] = np.frombuffer((b"ACG" * (L // 3 + 1))[:L], dtype=np.uint8)  # period 3: three distinct hashes
-            reads[3] = rng.choice(list(b"AC"), size=L).astype(np.uint8)           # low complexity
-            reads[4, : L // 2] = reads[4, L // 2: 2 * (L // 2)]                    # every k-mer of one half twice
-            got = mash.sketch_uniform(reads.reshape(-1), n, L, k, s)
-            rc, want = oracle.sketch_batch(reads.reshape(-1), synth.uniform_offsets(n, L), k, s, variant=1)
-            assert rc == 0
-            cnt = min(L - k, s)
-            assert np.array_equal(got, want[:, :cnt]), (knobs, k, s, L, n, [i for i in range(n) if not np.array_equal(got[i], want[i, :cnt])])
-    for name in ("PG_K2T_SEL_MUL", "PG_K2T_ROLLED", "PG_K2T_SEL_U"):
-        monkeypatch.delenv(name, raising=False)
+             (24, 5000, 30_000, 5), (32, 3, 9_000, 12), (11, 500, 2176 * 8 + 11 + 1, 6), (28, 300, 7_013, 8),
+             (21, 517, 539, 9), (21, 517, 1055, 9), (21, 733, 1487, 9), (21, 1185, 1207, 9), (21, 1746, 1_047_621, 5)]
+    for k, s, L, n in cases:
+        reads = rng.choice(list(b"ACGT"), size=n * L).astype(np.uint8).reshape(n, L)
+        reads[1] = ord("A")                                                   # homopolymer: one distinct hash
+        reads[2] = np.frombuffer((b"ACG" * (L // 3 + 1))[:L], dtype=np.uint8)  # period 3: three distinct hashes
+        reads[3] = rng.choice(list(b"AC"), size=L).astype(np.uint8)           # low complexity
+        reads[4, : L // 2] = reads[4, L // 2: 2 * (L // 2)]                    # every k-mer of one half twice
+        got = mash.sketch_uniform(reads.reshape(-1), n, L, k, s)
+        rc, want = oracle.sketch_batch(reads.reshape(-1), synth.uniform_offsets(n, L), k, s, variant=1)
+        assert rc == 0
+        cnt = min(L - k, s)
+        assert np.array_equal(got, want[:, :cnt]), (k, s, L, n, [i for i in range(n) if not np.array_equal(got[i], want[i, :cnt])])
     # ragged batch whose longest read spans several items: row x item mapping with empty items
     lens = [int(x) for x in rng.integers(1200, 50_000, 30)] + [0, 5, 1021, 1022, 1023]
     seqs = [bytes(rng.choice(list(b"ACGT"), size=l).astype(np.uint8)) for l in lens] + [b"T" * 30_000]

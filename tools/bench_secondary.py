@@ -19,7 +19,7 @@ ap.add_argument("--reads", type=int, default=100_000)
 ap.add_argument("--rows", type=int, default=512, help="row block of the all-pairs matrix to time")
 ap.add_argument("--primers", type=int, default=1_000_000)
 ap.add_argument("--iters", type=int, default=3)
-ap.add_argument("--only-k2", action="store_true", help="stop after the K2 legs (A/B runs with PG_K2_GENERIC=1)")
+ap.add_argument("--only-k2", action="store_true", help="stop after the K2 legs")
 args = ap.parse_args()
 
 L = _lib.lib()

@@ -1,7 +1,5 @@
-# One comprehensive GPU pass: parity tier, the driver's bench line, K2 A/B.  Every step is bounded.
+# One comprehensive GPU pass: parity tier, the bench line, the K2 timings.  Every step is bounded.
 set -x
 timeout 900 python -m pytest tests -m gpu -x -q --timeout 240 --timeout-method thread 2>&1 | tail -25
 timeout 600 python bench.py > gpurun_out/bench_n1.json 2> gpurun_out/bench_n1.err; tail -c 400 gpurun_out/bench_n1.err
 timeout 300 python tools/bench_secondary.py --only-k2 > gpurun_out/k2_thresh.jsonl 2>&1
-PG_K2_NO_THRESH=1 timeout 300 python tools/bench_secondary.py --only-k2 > gpurun_out/k2_nothresh.jsonl 2>&1
-cat gpurun_out/k2_thresh.jsonl gpurun_out/k2_nothresh.jsonl | cut -c1-300
